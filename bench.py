@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (this repo's CUDA path)
   python bench.py --impl reference --gpus N --steps K ...  (the reference's CPU algorithm on the host cores)
+  python bench.py ... --dump-outputs DIR                   (also writes the last timed tick's outputs, see dump_outputs)
 
 A "step" is one scheduler tick: tunable planner + DistroQueueInfo + utilization host allocator over every distro of
 the workload.  Headline workload (per GPU): configs[2] read per distro -- distro queues of 100 000 tasks each, Zipf
@@ -323,6 +324,37 @@ def time_resident(torch, eng, now, steps, warmup, stream):
     return e0.elapsed_time(e1) / steps
 
 
+DUMP_TASK_ROWS, DUMP_GROUP_ROWS, DUMP_DISTRO_ROWS = 1 << 20, 1 << 18, 1 << 16  # at most ~48 MB of float64 in all
+
+
+def dump_outputs(out_dir, po, ao):
+    """Write what Engine.download() returned for the last timed tick as DIR/<name>.npy (float64): the per-task order
+    and total value, every field of the per-distro queue info, per-group info and allocator result.  An output longer
+    than its row cap is cut to a fixed seeded sample of rows (the same rows on every run with the same arguments), so
+    two builds can be compared file for file.  Nanosecond sums above 2**53 are rounded to the nearest float64."""
+    os.makedirs(out_dir, exist_ok=True)
+
+    def rows(n, cap, seed):
+        return slice(None) if n <= cap else np.sort(np.random.default_rng(seed).choice(n, cap, replace=False))
+
+    def save(name, a):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+    def save_fields(prefix, a):
+        for f in a.dtype.names:
+            (save_fields if a.dtype[f].names else save)(f"{prefix}.{f}", a[f])
+
+    t = rows(po.order.shape[0], DUMP_TASK_ROWS, 1)
+    save("order", po.order[t])
+    save("total_value", po.total_value[t])
+    d = rows(po.info.shape[0], DUMP_DISTRO_ROWS, 2)
+    save_fields("queue_info", po.info[d])
+    save_fields("group_info", po.group_info[rows(po.group_info.shape[0], DUMP_GROUP_ROWS, 3)])
+    if ao is not None:
+        save_fields("alloc_result", ao.result[d])
+        save("alloc_status", ao.status[d])
+
+
 def measure_shapes(torch, eng, stream, peak, steps):
     """The other BASELINE shapes through the resident tick (same process, same engine)."""
     from evergreen_b200 import synth
@@ -422,7 +454,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-shapes", action="store_true")
     ap.add_argument("--no-delta", action="store_true", help="skip the resident-delta leg of the e2e object")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write rank 0's outputs of the last timed tick as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     args.block = max(1, min(args.block, args.distros))
     reps = max(1, args.distros // args.block)
@@ -515,6 +550,8 @@ def main():
     tasks_total = world * T
     value = tasks_total / (ms_per_step * 1e-3)
     po, ao = eng.download()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, po, ao)
     new_hosts_checksum = int(ao.result["new_hosts"].astype(np.int64).sum())
     order_ok = bool((np.sort(po.order[: args.tasks_per_distro]) == np.arange(args.tasks_per_distro)).all())
     H, G = hosts.n_hosts, distros.n_groups

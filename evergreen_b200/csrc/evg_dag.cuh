@@ -133,7 +133,8 @@ __global__ void __launch_bounds__(256) k_dag_group_pass(DDag X, const int32_t* _
   }
 }
 // bucket boundaries: unit_off[group_off[d] + g] = first position (distro-local) of group g in the sorted items;
-// the entry after a distro's last group is written by the host from grouped[d] (items that have a group)
+// the entry after a distro's last group is written by the host from grouped[d] (items that have a group); the entries of
+// groups no item is in keep the -1 they were set to, and the host gives them the start of the next group
 __global__ void __launch_bounds__(256) k_dag_units(DDag X, const int32_t* __restrict__ order, const int64_t* __restrict__ group_off,
                                                    int32_t* __restrict__ unit_off, int32_t* __restrict__ grouped) {
   const int64_t p = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;

@@ -831,7 +831,7 @@ struct evg_ctx {
   DevBuf b_taskoff, b_groupoff, b_cfg, b_gmax, b_unitbase;
   DevBuf b_hasdep, b_head, b_next, b_pslot, b_etask, b_elive, b_ca, b_crk, b_bestpair;
   DevBuf b_rn0, b_rn1, b_rn2, b_rn3, b_rn4, b_rn5, b_rn6, b_rn7;
-  DevBuf b_pf[36];  // evg_plan_from_finder: finder tables, candidate columns, compacted columns, edge scratch
+  DevBuf b_pf[39];  // evg_plan_from_finder: finder tables, candidate columns, compacted columns, edge scratch, group slots
   DevBuf b_err, b_dx0, b_dx1, b_dx2, b_dx3, b_dx4, b_dx5, b_dx6, b_dx7;
   DevBuf b_route, b_listW, b_listA, b_listB, b_listC, b_listG, b_listNA, b_listNB, b_listNC, b_unitv, b_unita, b_unitn, b_unitmask;
   DevBuf b_punt, b_puntcnt;
@@ -2171,10 +2171,26 @@ struct PfCols {  // nine planner columns, candidate table (src) and compacted ta
   int32_t *o_priority, *o_numdep, *o_tgo, *o_gid, *o_vid;
   uint32_t* o_flags;
   int64_t *o_expected, *o_qbasis, *o_wbasis;
+  const int64_t* group_off;  // candidate group table (n_distros + 1); nullptr when no distro has a group
+  const int32_t* group_remap;  // [group_off[d] + g] = distro-local slot of candidate group g among the kept groups
 };
+// used[group_off[d] + g] = 1 for every candidate group g of distro d that kept at least one task; a group id outside
+// [-1, groups of the distro) raises err[1] instead of indexing anything.
+__global__ void __launch_bounds__(256) k_pf_mark_groups(int64_t n_cand, int32_t D, const int64_t* __restrict__ cand_off,
+                                                        const int32_t* __restrict__ kept, const int64_t* __restrict__ count,
+                                                        const int32_t* __restrict__ gid, const int64_t* __restrict__ group_off,
+                                                        uint8_t* __restrict__ used, int* err) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  const int d = block_find_distro(cand_off, D, i, n_cand);
+  if (d < 0 || i - cand_off[d] >= count[d]) return;
+  const int32_t g = gid[cand_off[d] + kept[i]];
+  if (g < -1 || g >= group_off[d + 1] - group_off[d]) atomicOr(err + 1, 1);
+  else if (g >= 0) used[group_off[d] + g] = 1;
+}
 // One thread per KEPT task: its row of the candidate table moves to its place in the compacted table; the
 // EVG_TF_DEPS_MET bit and the stamped wait basis come from the device's own evaluation (k_deps_met), like
-// evg_upload_with_deps.  new_idx[candidate row] = distro-local index in the compacted queue (memset to -1 before).
+// evg_upload_with_deps; the group id becomes the group's slot among the groups that kept a task.
+// new_idx[candidate row] = distro-local index in the compacted queue (memset to -1 before).
 __global__ void __launch_bounds__(256) k_pf_gather(int64_t n_new, int32_t D, const int64_t* __restrict__ new_off, const int64_t* __restrict__ cand_off,
                                                    const int32_t* __restrict__ kept, PfCols C, const uint8_t* __restrict__ met,
                                                    const int64_t* __restrict__ met_time, int32_t* __restrict__ new_idx, int64_t* __restrict__ src_row) {
@@ -2183,7 +2199,9 @@ __global__ void __launch_bounds__(256) k_pf_gather(int64_t n_new, int32_t D, con
   if (d < 0) return;
   const int64_t k = i - new_off[d];
   const int64_t src = cand_off[d] + kept[cand_off[d] + k];
-  C.o_priority[i] = C.priority[src]; C.o_numdep[i] = C.numdep[src]; C.o_tgo[i] = C.tgo[src]; C.o_gid[i] = C.gid[src]; C.o_vid[i] = C.vid[src];
+  const int32_t g = C.gid[src];
+  C.o_priority[i] = C.priority[src]; C.o_numdep[i] = C.numdep[src]; C.o_tgo[i] = C.tgo[src]; C.o_vid[i] = C.vid[src];
+  C.o_gid[i] = (g >= 0 && C.group_remap) ? C.group_remap[C.group_off[d] + g] : g;
   C.o_expected[i] = C.expected[src]; C.o_qbasis[i] = C.qbasis[src];
   C.o_flags[i] = (C.flags[src] & ~EVG_TF_DEPS_MET) | ((met[src] & 1) ? EVG_TF_DEPS_MET : 0u);
   const int64_t wb = C.wbasis[src], st = met_time[src];
@@ -2303,6 +2321,49 @@ int evg_plan_from_finder(evg_ctx* c, const evg_runnable_in* in, const evg_task_s
                 !cand->task_group_order || !cand->group_id || !cand->version_id || !cand->flags))
     return fail(EVG_ERR_INVALID, "null candidate column");
   if (E > 0 && (!cand->dep_off || !cand->dep_idx)) return fail(EVG_ERR_INVALID, "null candidate dependency edges");
+  if (!distros->group_off || distros->group_off[0] != 0) return fail(EVG_ERR_INVALID, "null or misplaced group_off");
+  for (int32_t d = 0; d < D; d++)
+    if (distros->group_off[d + 1] < distros->group_off[d]) return fail(EVG_ERR_INVALID, "group offsets of distro %d decrease", d);
+  const int64_t Gc = distros->group_off[D];
+  if (Gc > 0 && !distros->group_max_hosts) return fail(EVG_ERR_INVALID, "null group_max_hosts");
+  // Group slots of the resident tick are the candidate groups that kept a task, in id order (include/evg_sched.h): a
+  // group the finder emptied must not come back as a TaskGroupInfo, the reference builds those from the plan's tasks
+  // alone (scheduler.go:60-143).  remap[group_off[d] + g] = new slot of candidate group g, -1 when it kept nothing.
+  std::vector<int64_t> kgroup_off(size_t(D) + 1, 0);
+  std::vector<int32_t> kgroup_max, remap(size_t(Gc), -1), host_gid;
+  evg_host_soa hosts_k;
+  const evg_host_soa* hosts_in = hosts;
+  auto keep_groups = [&](const std::vector<uint8_t>& used) {
+    for (int32_t d = 0; d < D; d++) {
+      int32_t k = 0;
+      for (int64_t g = distros->group_off[d]; g < distros->group_off[d + 1]; g++)
+        if (used[size_t(g)]) { remap[size_t(g)] = k++; kgroup_max.push_back(distros->group_max_hosts[g]); }
+      kgroup_off[size_t(d) + 1] = kgroup_off[size_t(d)] + k;
+    }
+    // hosts name groups by candidate slot; a host running a task of an emptied group is in no queued group
+    // (groupByTaskGroup gives its bucket no TaskGroupInfo, utilization_based_host_allocator.go:223-260).  Malformed host
+    // tables are left for upload_hosts to reject.
+    if (!hosts || Gc == 0 || hosts->n_hosts <= 0 || !hosts->group_id || !host_off || host_off[0] != 0 || host_off[D] != hosts->n_hosts) return;
+    for (int32_t d = 0; d < D; d++)
+      if (host_off[d + 1] < host_off[d]) return;
+    host_gid.assign(hosts->group_id, hosts->group_id + hosts->n_hosts);
+    for (int32_t d = 0; d < D; d++) {
+      const int64_t g0 = distros->group_off[d], ng = distros->group_off[d + 1] - g0;
+      for (int64_t h = host_off[d]; h < host_off[d + 1]; h++) {
+        const int32_t g = host_gid[size_t(h)];
+        if (g >= 0 && g < ng) host_gid[size_t(h)] = remap[size_t(g0 + g)] >= 0 ? remap[size_t(g0 + g)] : EVG_HG_UNQUEUED;
+      }
+    }
+    hosts_k = *hosts;
+    hosts_k.group_id = host_gid.data();
+    hosts_in = &hosts_k;
+  };
+  auto kept_table = [&]() {
+    evg_distro_table dn = *distros;
+    dn.group_off = kgroup_off.data();
+    dn.group_max_hosts = kgroup_max.empty() ? nullptr : kgroup_max.data();
+    return dn;
+  };
   CK(cudaSetDevice(c->device));
   cudaStream_t s = c->stream;
   CK(c->b_err.ensure(sizeof(int) * 4));
@@ -2311,7 +2372,9 @@ int evg_plan_from_finder(evg_ctx* c, const evg_runnable_in* in, const evg_task_s
   c->have_tasks = false;
   if (T == 0) {
     for (int32_t d = 0; d < D; d++) count[d] = 0;
-    return evg_upload(c, cand, distros, hosts, host_off, acfg);
+    keep_groups(std::vector<uint8_t>(size_t(Gc), 0));
+    const evg_distro_table dn = kept_table();
+    return evg_upload(c, cand, &dn, hosts_in, host_off, acfg);
   }
   // 1. Task.DependenciesMet / AllDependenciesSatisfied of every candidate, with the DependenciesMetTime stamps
   int rc = deps_to_device(c, in->deps, 1, dep_finished_ns, now_ns, /*want_stamp=*/true);
@@ -2338,25 +2401,38 @@ int evg_plan_from_finder(evg_ctx* c, const evg_runnable_in* in, const evg_task_s
   r.finder = c->b_pf[6].as<uint8_t>(); r.met = c->b_dx7.as<uint8_t>();
   k_runnable<<<unsigned(D), 256, 0, s>>>(r, c->b_pf[7].as<int32_t>(), c->b_pf[8].as<int64_t>(), c->b_err.as<int>());
   c->launches++;
+  UPF(c->b_pf[12], cand->group_id, T, int32_t);
+  std::vector<uint8_t> used(size_t(Gc), 0);
+  if (Gc > 0) {  // which candidate groups kept a task
+    UPF(c->b_pf[36], distros->group_off, D + 1, int64_t);
+    CK(c->b_pf[37].ensure(size_t(Gc)));
+    CK(cudaMemsetAsync(c->b_pf[37].p, 0, size_t(Gc), s));
+    k_pf_mark_groups<<<grid_for(T, 256), 256, 0, s>>>(T, D, c->b_pf[0].as<int64_t>(), c->b_pf[7].as<int32_t>(), c->b_pf[8].as<int64_t>(),
+                                                      c->b_pf[12].as<int32_t>(), c->b_pf[36].as<int64_t>(), c->b_pf[37].as<uint8_t>(),
+                                                      c->b_err.as<int>());
+    c->launches++;
+  }
   CK(cudaGetLastError());
-  // 3. the only thing the host needs before the planner can be routed: how many tasks each distro kept
-  int bad = 0;
+  // 3. the only things the host needs before the planner can be routed: how many tasks each distro kept, and which groups
+  int bad[2] = {0, 0};
   CK(cudaMemcpyAsync(count, c->b_pf[8].p, sizeof(int64_t) * size_t(D), cudaMemcpyDeviceToHost, s));
-  CK(cudaMemcpyAsync(&bad, c->b_err.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+  CK(cudaMemcpyAsync(bad, c->b_err.p, sizeof(bad), cudaMemcpyDeviceToHost, s));
+  if (Gc > 0) CK(cudaMemcpyAsync(used.data(), c->b_pf[37].p, size_t(Gc), cudaMemcpyDeviceToHost, s));
   if (runnable) CK(cudaMemcpyAsync(runnable, c->b_pf[7].p, sizeof(int32_t) * size_t(T), cudaMemcpyDeviceToHost, s));
   CK(cudaStreamSynchronize(s));
-  if (bad) return fail(EVG_ERR_INVALID, "a project row or dep_ref is out of range");
+  if (bad[0]) return fail(EVG_ERR_INVALID, "a project row or dep_ref is out of range");
+  if (bad[1]) return fail(EVG_ERR_INVALID, "a kept candidate's group_id is out of range for its distro");
   std::vector<int64_t> new_off(size_t(D) + 1, 0);
   for (int32_t d = 0; d < D; d++) {
     if (count[d] < 0 || count[d] > in->task_off[d + 1] - in->task_off[d]) return fail(EVG_ERR_CUDA, "finder count out of range");
     new_off[size_t(d) + 1] = new_off[size_t(d)] + count[d];
   }
   const int64_t Tn = new_off[size_t(D)];
+  keep_groups(used);
   // 4. candidate columns to the device, compaction into the context's own buffers
   UPF(c->b_pf[9], cand->priority, T, int32_t);
   UPF(c->b_pf[10], cand->num_dependents, T, int32_t);
   UPF(c->b_pf[11], cand->task_group_order, T, int32_t);
-  UPF(c->b_pf[12], cand->group_id, T, int32_t);
   UPF(c->b_pf[13], cand->version_id, T, int32_t);
   UPF(c->b_pf[14], cand->flags, T, uint32_t);
   UPF(c->b_pf[15], cand->expected_ns, T, int64_t);
@@ -2377,6 +2453,11 @@ int evg_plan_from_finder(evg_ctx* c, const evg_runnable_in* in, const evg_task_s
   pc.o_priority = c->b_pf[19].as<int32_t>(); pc.o_numdep = c->b_pf[20].as<int32_t>(); pc.o_tgo = c->b_pf[21].as<int32_t>();
   pc.o_gid = c->b_pf[22].as<int32_t>(); pc.o_vid = c->b_pf[23].as<int32_t>(); pc.o_flags = c->b_pf[24].as<uint32_t>();
   pc.o_expected = c->b_pf[25].as<int64_t>(); pc.o_qbasis = c->b_pf[26].as<int64_t>(); pc.o_wbasis = c->b_pf[27].as<int64_t>();
+  pc.group_off = nullptr; pc.group_remap = nullptr;
+  if (Gc > 0) {
+    UPF(c->b_pf[38], remap.data(), Gc, int32_t);
+    pc.group_off = c->b_pf[36].as<int64_t>(); pc.group_remap = c->b_pf[38].as<int32_t>();
+  }
   const int64_t* d_new_off = c->b_pf[18].as<int64_t>();
   const int64_t* d_cand_off = c->b_pf[0].as<int64_t>();
   if (Tn > 0) {
@@ -2424,12 +2505,12 @@ int evg_plan_from_finder(evg_ctx* c, const evg_runnable_in* in, const evg_task_s
   ts.priority = pc.o_priority; ts.num_dependents = pc.o_numdep; ts.task_group_order = pc.o_tgo; ts.group_id = pc.o_gid; ts.version_id = pc.o_vid;
   ts.flags = pc.o_flags; ts.expected_ns = pc.o_expected; ts.queue_basis_ns = pc.o_qbasis; ts.wait_basis_ns = pc.o_wbasis;
   if (En > 0) { ts.dep_off = c->b_pf[33].as<int64_t>(); ts.dep_idx = c->b_pf[35].as<int32_t>(); }
-  evg_distro_table dn = *distros;
+  evg_distro_table dn = kept_table();
   dn.task_off = new_off.data();
   rc = upload_tasks(c, &ts, &dn, /*copy_columns=*/false, /*adopt=*/true, (En > 0) ? edge_off.data() : nullptr);
   if (rc != EVG_OK) return rc;
   if (hosts) {
-    rc = upload_hosts(c, hosts, host_off, acfg, D);
+    rc = upload_hosts(c, hosts_in, host_off, acfg, D);
     if (rc != EVG_OK) return rc;
   }
   CK(cudaStreamSynchronize(s));
@@ -2625,6 +2706,13 @@ int evg_dag_rebuild_batch(evg_ctx* c, const evg_dag_in* in, const int64_t* item_
     max_n = std::max(max_n, item_off[d + 1] - item_off[d]);
   }
   if (max_n >= (int64_t(1) << 31) - 1) return fail(EVG_ERR_INVALID, "a queue exceeds 2^31 items");
+  // k_dag_units writes unit_off[group_off[d] + d + group_id]: every id must name one of its distro's groups
+  for (int32_t d = 0; d < D; d++) {
+    const int64_t ng = group_off[d + 1] - group_off[d];
+    for (int64_t i = item_off[d]; i < item_off[d + 1]; i++)
+      if (in->group_id[i] < -1 || in->group_id[i] >= ng)
+        return fail(EVG_ERR_INVALID, "item %lld: group_id %d outside [-1, %lld) of distro %d", (long long)i, int(in->group_id[i]), (long long)ng, d);
+  }
   const int64_t G = group_off[D];
   CK(cudaSetDevice(c->device));
   cudaStream_t s = c->stream;
@@ -2673,6 +2761,7 @@ int evg_dag_rebuild_batch(evg_ctx* c, const evg_dag_in* in, const int64_t* item_
       LAUNCH(c, k_dag_group_pass, grid_for(N, 256), 256, x, buf[cur], buf[cur ^ 1], L);
       cur ^= 1;
     }
+    CK(cudaMemsetAsync(c->b_rn7.p, 0xFF, sizeof(int32_t) * size_t(G + D), s));  // -1: a group no item is in
     LAUNCH(c, k_dag_units, grid_for(N, 256), 256, x, buf[cur], c->b_groupoff.as<int64_t>(), c->b_rn7.as<int32_t>(), d_grouped);
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(unit_items, buf[cur], sizeof(int32_t) * size_t(N), cudaMemcpyDeviceToHost, s));
@@ -2682,7 +2771,15 @@ int evg_dag_rebuild_batch(evg_ctx* c, const evg_dag_in* in, const int64_t* item_
   CK(cudaMemcpyAsync(n_sorted, d_nsorted, sizeof(int32_t) * size_t(D), cudaMemcpyDeviceToHost, s));
   CK(cudaMemcpyAsync(n_cycles, d_ncycles, sizeof(int32_t) * size_t(D), cudaMemcpyDeviceToHost, s));
   CK(cudaStreamSynchronize(s));
-  for (int32_t d = 0; d < D; d++) unit_off[group_off[d + 1] + d] = grouped[size_t(d)];  // the closing entry of each distro
+  if (N == 0) std::fill(unit_off, unit_off + (G + D), -1);
+  for (int32_t d = 0; d < D; d++) {
+    int32_t* u = unit_off + group_off[d] + d;
+    const int64_t ng = group_off[d + 1] - group_off[d];
+    u[ng] = grouped[size_t(d)];  // the closing entry of each distro
+    // a group without items is the empty range that starts where the next group starts
+    for (int64_t g = ng - 1; g >= 0; g--)
+      if (u[g] < 0) u[g] = u[g + 1];
+  }
   return EVG_OK;
 }
 

@@ -269,7 +269,9 @@ class Engine:
     def plan_from_finder(self, table: "S.RunnableTable", candidates: S.TaskSoA, distros: S.DistroTable,
                          hosts: Optional[S.HostSoA], dep_finished: Optional[np.ndarray], now: int):
         """evg_plan_from_finder: finder -> dependency predicate -> compaction -> resident planner inputs on the device.
-        -> (runnable, count) as find_runnable_batch; the context then holds the tick of the KEPT tasks (run / download)."""
+        -> (runnable, count) as find_runnable_batch; the context then holds the tick of the KEPT tasks (run / download).
+        Its group slots are the candidate groups that kept a task: `self.group_slots` lists them as rows of the
+        candidate distro table, `self.group_slot_off` cuts that list per distro (see kept_group_slots)."""
         if table.deps is None:
             raise ValueError("plan_from_finder needs the candidates' dependency table")
         runnable = self._out("runnable", table.n_tasks, np.int32)
@@ -285,7 +287,9 @@ class Engine:
                                               L.ptr(fin) if fin is not None and fin.shape[0] else None, int(now),
                                               L.ptr(runnable) if table.n_tasks else None, L.ptr(count) if table.n_distros else None))
         del keep
-        self._n_tasks, self._n_distros, self._n_groups = int(count.sum()), distros.n_distros, distros.n_groups
+        self.group_slots, self.group_slot_off = kept_group_slots(table.task_off, runnable, count, candidates.group_id,
+                                                                 distros.group_off)
+        self._n_tasks, self._n_distros, self._n_groups = int(count.sum()), distros.n_distros, int(self.group_slot_off[-1])
         self._has_hosts = hosts is not None
         return runnable, count
 
@@ -333,6 +337,22 @@ class Engine:
                                          L.ptr(ginfo) if ginfo.shape[0] else None, L.ptr(group_off), D, int(now),
                                          C.byref(as_)))
         return ao, ginfo
+
+
+def kept_group_slots(task_off, runnable, count, group_id, group_off):
+    """The group slots evg_plan_from_finder leaves resident (include/evg_sched.h): per distro, the candidate groups
+    that kept at least one task, in id order.  -> (their rows in the candidate distro table, offsets per distro)."""
+    task_off, group_off = np.asarray(task_off, np.int64), np.asarray(group_off, np.int64)
+    D, T = int(task_off.shape[0]) - 1, int(task_off[-1])
+    used = np.zeros(int(group_off[-1]), dtype=bool)
+    if T > 0 and used.shape[0] > 0:
+        dist = np.repeat(np.arange(D), np.diff(task_off))
+        kept = (np.arange(T) - task_off[dist]) < np.asarray(count, np.int64)[dist]
+        g = np.asarray(group_id)[task_off[dist[kept]] + np.asarray(runnable)[kept]]
+        live = g >= 0
+        used[group_off[dist[kept][live]] + g[live]] = True
+    slots = np.nonzero(used)[0]
+    return slots, np.searchsorted(slots, group_off).astype(np.int64)
 
 
 _default_engine: Optional[Engine] = None
@@ -435,19 +455,22 @@ def persist_task_queues(batch: Sequence[Tuple[M.Distro, List[M.Task]]], now: int
     for d, (distro, tasks) in enumerate(batch):
         ga, gb = int(table.group_off[d]), int(table.group_off[d + 1])
         info = _queue_info_from_rows(po.info[d], po.group_info[ga:gb], keys[d].group_names)
+        incl = distro.dispatcher_settings.version == M.DISPATCHER_VERSION_REVISED_WITH_DEPENDENCIES
         queue = []
         for row in items[int(item_off[d]):int(item_off[d + 1])]:
             t = tasks[int(row["task"])]
-            t.expected_duration = int(row["expected_ns"])
+            met = bool(int(row["flags"]) & L.EVG_QI_DEPS_MET)
+            if met or not incl:  # GetDistroQueueInfo stamps ExpectedDuration only on the tasks it counts (scheduler.go:98)
+                t.expected_duration = int(row["expected_ns"])
             t.sorting_value_breakdown = M.SortingValueBreakdown(total_value=int(row["total_value"]))
             queue.append(M.TaskQueueItem(
                 id=t.id, display_name=t.display_name, build_variant=t.build_variant,
                 revision_order_number=t.revision_order_number, requester=t.requester, revision=t.revision, project=t.project,
-                expected_duration=int(row["expected_ns"]), priority=int(row["priority"]),
+                expected_duration=t.expected_duration, priority=int(row["priority"]),
                 sorting_value_breakdown=t.sorting_value_breakdown, group=t.task_group,
                 group_max_hosts=t.task_group_max_hosts, group_index=int(row["group_index"]), version=t.version,
                 activated_by=t.activated_by, dependencies=[dep.task_id for dep in t.depends_on],
-                dependencies_met=bool(int(row["flags"]) & L.EVG_QI_DEPS_MET)))
+                dependencies_met=met))
         for t in tasks:  # SetTasksScheduledAndDepsMetTime (model/task/task.go:1164-1195), every prioritised task
             if M.is_zero_time(t.scheduled_time):
                 t.scheduled_time = now
@@ -551,7 +574,8 @@ def plan_candidates(batch: Sequence[Tuple[M.Distro, List[M.Task]]], project_refs
     """The finder -> checkDependenciesMet -> PrioritizeTasks hand-over of scheduler.PlanDistro (wrapper.go:60-118,
     scheduler.go:56-168) without the host in the middle: `batch` holds every distro's CANDIDATES; the device filters them,
     evaluates their dependencies, compacts the planner's columns and plans (evg_plan_from_finder).  Returns, per distro,
-    (ranked kept tasks with TotalValue stamped, DistroQueueInfo)."""
+    (ranked kept tasks with TotalValue stamped, DistroQueueInfo); the TaskGroupInfos are those of the groups that kept a
+    task, group slot k naming the k-th such candidate group."""
     eng = engine or default_engine()
     table = S.marshal_runnable(batch, project_refs, finder, dependency_db)
     if table.deps is None:
@@ -570,8 +594,9 @@ def plan_candidates(batch: Sequence[Tuple[M.Distro, List[M.Task]]], project_refs
             t.sorting_value_breakdown = M.SortingValueBreakdown(total_value=int(po.total_value[r]))
             ranked.append(t)
         a_new += len(kept)
-        ga, gb = int(dtable.group_off[d]), int(dtable.group_off[d + 1])
-        out.append((ranked, _queue_info_from_rows(po.info[d], po.group_info[ga:gb], keys[d].group_names)))
+        ga, gb = int(eng.group_slot_off[d]), int(eng.group_slot_off[d + 1])
+        names = [keys[d].group_names[int(g - dtable.group_off[d])] for g in eng.group_slots[ga:gb]]
+        out.append((ranked, _queue_info_from_rows(po.info[d], po.group_info[ga:gb], names)))
     return out
 
 

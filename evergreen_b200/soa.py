@@ -211,7 +211,7 @@ def dependencies_met(t: M.Task, in_queue: Dict[str, M.Task], db: Optional[Dict[s
             dep_task = db.get(dep.task_id)
         if dep_task is None:
             return False
-        if not satisfies_dependency(dep, dep_task):
+        if not satisfies_dependency(next(x for x in t.depends_on if x.task_id == dep.task_id), dep_task):  # the first one naming it
             return False
     if now is not None:
         best = M.ZERO_TIME
@@ -502,8 +502,10 @@ def marshal_deps(batch: Sequence[tuple], dependency_db: Optional[Dict[str, M.Tas
             tstate.append(_task_state(t))
             pre.append((L.EVG_TP_OVERRIDE if t.override_dependencies else 0) |
                        (0 if M.is_zero_time(t.dependencies_met_time) else L.EVG_TP_MET_TIME))
+            first: Dict[str, str] = {}
             for d in t.depends_on:
-                want.append(_want(d.status))
+                # SatisfiesDependency judges a dependency task by the FIRST Dependency naming it (task.go:529-543)
+                want.append(_want(first.setdefault(d.task_id, d.status)))
                 j = index.get(d.task_id)
                 if j is not None:
                     kind.append(L.EVG_DEP_IN_QUEUE); ref.append(base + j)

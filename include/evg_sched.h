@@ -307,7 +307,8 @@ typedef struct {
   int32_t group_max_hosts; /* GroupMaxHosts = Task.TaskGroupMaxHosts (0 outside task groups) */
   uint32_t flags;          /* EVG_QI_* */
   int64_t priority;        /* Priority */
-  int64_t expected_ns;     /* ExpectedDuration as GetDistroQueueInfo left it (scheduler.go:98) */
+  int64_t expected_ns;     /* FetchExpectedDuration().Average: the ExpectedDuration GetDistroQueueInfo writes on every task it
+                              counts (scheduler.go:98); under IncludesDependencies a task without EVG_QI_DEPS_MET keeps its own */
   int64_t total_value;     /* SortingValueBreakdown.TotalValue of the unit the task was emitted from (planner.go:475) */
 } evg_queue_item;
 #define EVG_PERSISTED_QUEUE_CAP 10000 /* TaskQueue.Save keeps the first 10 000 items (model/task_queue.go:216-219) */
@@ -369,7 +370,8 @@ typedef struct {
   const int64_t* dep_off;   /* n_tasks + 1 */
   const uint8_t* dep_kind;  /* EVG_DEP_* */
   const int32_t* dep_ref;
-  const uint8_t* dep_want;  /* EVG_WANT_* */
+  const uint8_t* dep_want;  /* EVG_WANT_* of the FIRST of the task's Dependencies naming the same task: SatisfiesDependency
+                              judges every edge to a task by that one (model/task/task.go:529-543) */
   const uint8_t* task_state;/* n_tasks, EVG_TS_* of the in-queue tasks themselves */
   const uint8_t* task_pre;  /* n_tasks, EVG_TP_* */
   const uint8_t* ext_state; /* n_ext, EVG_TS_* */
@@ -448,8 +450,12 @@ int evg_find_runnable_batch(evg_ctx* ctx, const evg_runnable_in* in, int32_t* ru
  * -> a stable compaction of the nine planner columns (EVG_TF_DEPS_MET and the stamped wait basis applied on the way)
  * -> the dependency edges whose two ends were kept, re-indexed.  The compacted table becomes the context's resident
  * tick: call evg_run_resident / evg_download next; ranks refer to the compacted queues, and `runnable` (n_tasks, may be
- * NULL) / `count` (n_distros) map them back exactly as evg_find_runnable_batch reports them.  The only values the host
- * reads in between are the n_distros counts (the routing needs queue lengths).
+ * NULL) / `count` (n_distros) map them back exactly as evg_find_runnable_batch reports them.  Group slot k of distro d
+ * in the resident tick -- its evg_group_info row and a queue item's group_max_hosts -- is the k-th candidate group of d,
+ * in id order, that kept at least one task; a group the finder emptied has no slot and no TaskGroupInfo, as in the
+ * reference, which builds them from the planned tasks (scheduler.go:60-143).  hosts->group_id names candidate groups;
+ * a host running a task of an emptied group counts as EVG_HG_UNQUEUED.  The only values the host reads in between are
+ * the n_distros counts and one byte per candidate group (the routing needs queue lengths and group counts).
  * Replaces: the finder + checkDependenciesMet + PrioritizeTasks hand-over inside scheduler.PlanDistro
  * (scheduler/wrapper.go:60-118, scheduler/scheduler.go:56-168), where the filtered []task.Task is rebuilt on the host. */
 int evg_plan_from_finder(evg_ctx* ctx, const evg_runnable_in* in, const evg_task_soa* candidates, const evg_distro_table* distros,
@@ -592,8 +598,11 @@ typedef struct {
  *   cyclic component, n_cycles[d] of them); the rest of the distro's slots are -2.
  * unit_items[item_off[d] ..] = the items that have a group, bucketed by group id and stably sorted by GroupIndex inside
  *   each bucket (d.taskGroups[...].tasks); group g of distro d is unit_items[item_off[d] + unit_off[u + g] ..
- *   item_off[d] + unit_off[u + g + 1]) with u = group_off[d] + d (each distro has one closing entry).
- * Host pointers.  group_off (n_distros + 1) counts the groups of each distro. */
+ *   item_off[d] + unit_off[u + g + 1]) with u = group_off[d] + d (each distro has one closing entry).  A declared
+ *   group no item is in is the empty range that starts where the next group starts.
+ * Host pointers.  group_off (n_distros + 1) counts the groups of each distro; unit_off holds group_off[n_distros] +
+ * n_distros entries.  Every group_id must be -1 or below its distro's group count: -EVG_ERR_INVALID otherwise, checked
+ * on the host before anything is copied or launched. */
 int evg_dag_rebuild_batch(evg_ctx* ctx, const evg_dag_in* in, const int64_t* item_off, const int64_t* group_off, int32_t n_distros,
                           int32_t* sorted, int32_t* n_sorted, int32_t* n_cycles, int32_t* unit_items, int32_t* unit_off);
 

@@ -306,6 +306,8 @@ std::vector<uint8_t> deps_met(const View& v) {
     for (int64_t e = e0; e < e1 && ok; e++) {
       std::string_view dep_id = sv(t.dep_task_id, e);
       std::string_view dep_status, want = sv(t.dep_status, e);
+      for (int64_t f = e0; f < e; f++)  // SatisfiesDependency reads the FIRST Dependency naming the task (task.go:529-543)
+        if (sv(t.dep_task_id, f) == dep_id) { want = sv(t.dep_status, f); break; }
       bool dep_blocked = false;
       auto it = cache.find(dep_id);
       if (it != cache.end()) {

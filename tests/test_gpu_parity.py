@@ -919,9 +919,9 @@ def test_planner_consumes_the_finders_device_output(engine, finder):
         for f in ("length", "length_with_dependencies_met", "count_dep_filled_merge_queue_tasks", "expected_duration",
                   "max_duration_threshold", "count_duration_over_threshold", "duration_over_threshold", "count_wait_over_threshold"):
             assert getattr(gi, f) == getattr(wi, f), f
-        live = lambda infos: sorted((g.name, g.count, g.expected_duration, g.count_duration_over_threshold, g.count_wait_over_threshold)  # noqa: E731
-                                    for g in infos if g.count or g.name == "")
-        assert live(gi.task_group_infos) == live(wi.task_group_infos)
+        every = lambda infos: sorted((g.name, g.count, g.max_hosts, g.expected_duration, g.count_duration_over_threshold,  # noqa: E731
+                                      g.count_wait_over_threshold) for g in infos)
+        assert every(gi.task_group_infos) == every(wi.task_group_infos)
     assert 2000 < n_kept < sum(len(t) for _, t in batch)
 
 

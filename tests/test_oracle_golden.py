@@ -1,5 +1,6 @@
 """The oracle (oracle/evg_oracle.cpp) against every known answer the
 reference's own tests hold for this path (SURVEY.md §8c).  CPU only."""
+import copy
 import itertools
 
 import pytest
@@ -277,3 +278,50 @@ def test_dependencies_met_cases(case):
 def test_blocked_cases(case):
     t = M.Task(id="t1", depends_on=[M.Dependency(task_id="", unattainable=u) for u in case["unattainable"]])
     assert t.blocked() == case["expect"]
+
+
+# ---------------------------------------------------------------- PersistTaskQueue (scheduler/task_queue_persister_test.go)
+def test_task_queue_persister_golden():
+    """TestDBTaskQueuePersister: the persisted items of the two queues, their fields copied from the tasks, t5's
+    ExpectedDuration the ten-minute default, and the two queue infos the test checks first."""
+    from oracle import oracle_persist as OP
+    g = G.load("task_queue_persister.json")
+    now = 10 ** 18
+    for q in g["queues"]:
+        src = {t["id"]: t for t in g["tasks"]}
+        tasks = [G.make_task(src[i], now, 0) for i in q["tasks"]]
+        info = O.queue_info(q["distro"], [G.make_task(src[i], now, 0) for i in q["tasks"]], g["max_duration_threshold_ns"], False, now)
+        assert (info.length, info.length_with_dependencies_met) == (q["length"], q["length_with_dependencies_met"]), q["ref"]
+        items = OP.saved_queue(OP.task_queue_items(OP.stamp_planned_tasks(tasks, False, now)))
+        assert [it.id for it in items] == q["tasks"], q["ref"]
+        assert [it.expected_duration for it in items] == q["expected_durations"], q["ref"]
+        for it in items:
+            s = src[it.id]
+            assert (it.display_name, it.build_variant, it.revision_order_number, it.requester, it.revision, it.project,
+                    it.activated_by) == (s["display_name"], s["build_variant"], s["revision_order_number"], s["requester"],
+                                         s["revision"], s["project"], s["activated_by"])
+            assert it.dependencies == [d["task_id"] for d in s.get("depends_on", [])]
+            assert it.dependencies_met == (not s.get("depends_on"))  # "someTask" does not exist: never met
+    # Save keeps 10 000 items; the projection itself keeps every task
+    many = [M.Task(id=f"t{k}") for k in range(10001)]
+    assert len(OP.task_queue_items(many)) == 10001 and [it.id for it in OP.saved_queue(OP.task_queue_items(many))] == [t.id for t in many[:10000]]
+
+
+def test_persister_restatement_stamps_like_get_distro_queue_info():
+    """GetDistroQueueInfo's writes the persisted items read: a fresh met verdict stamps DependenciesMetTime (latest
+    FinishedAt, else now), an earlier stamp is kept, and under IncludesDependencies a task whose dependencies are not
+    met keeps its own ExpectedDuration."""
+    from oracle import oracle_persist as OP
+    now, MIN = 10 ** 18, 60 * 10 ** 9
+    db = {"ok": M.Task(id="ok", status="success"), "bad": M.Task(id="bad", status="failed")}
+    mk = lambda i, **kw: M.Task(id=i, expected_duration=0, **kw)  # noqa: E731
+    tasks = [mk("a", depends_on=[M.Dependency("ok", finished_at=now - 5 * MIN), M.Dependency("ok", finished_at=now - 9 * MIN)]),
+             mk("b", depends_on=[M.Dependency("ok")]),
+             mk("c", depends_on=[M.Dependency("bad")]),
+             mk("d", depends_on=[M.Dependency("bad")], dependencies_met_time=now - MIN),
+             mk("e", depends_on=[M.Dependency("bad")], override_dependencies=True)]
+    for incl in (False, True):
+        ts = OP.stamp_planned_tasks(copy.deepcopy(tasks), incl, now, db)
+        assert [t.dependencies_met_time for t in ts] == [now - 5 * MIN, now, M.ZERO_TIME, now - MIN, M.ZERO_TIME]
+        assert [it.dependencies_met for it in OP.task_queue_items(ts)] == [True, True, False, True, True]
+        assert [t.expected_duration for t in ts] == [10 * MIN, 10 * MIN, 0 if incl else 10 * MIN, 10 * MIN, 10 * MIN]

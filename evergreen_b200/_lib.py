@@ -181,6 +181,8 @@ SYMBOLS = {
     "evg_run_resident": (C.c_int, [_P, C.c_int64, C.c_uint32]),
     "evg_download": (C.c_int, [_P, _P, _P]),
     "evg_download_queue": (C.c_int, [_P, C.c_int32, _P, _P, C.c_int64]),
+    "evg_run_resident_head": (C.c_int, [_P, C.c_int64, C.c_uint32, C.c_int32]),
+    "evg_download_queue_bd": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_int64]),
     "evg_device_result_ptr": (_P, [_P]),
     "evg_bind_result_buffer": (C.c_int, [_P, _P, C.c_int64]),
     "evg_last_launch_count": (C.c_int64, [_P]),

@@ -991,3 +991,301 @@ __global__ void __launch_bounds__(256) k_gemit(DDistros D, DGen G, int32_t* __re
     total_value[p] = unord_i64(vmax_ord - key);
   }
 }
+
+// ---- the persisted head (evg_run_resident_head): only the first min(length, cap) ranks of every general-path distro ----
+// After k_gplace the (key, index) pairs of a distro sit in key_lo[0] / key_hi[0] / idx[0] in canonical tie order, so the
+// first cap ranks of the stable sort are the pairs with the cap smallest keys, ties broken by buffer position:
+//   k_hinit/k_hhist/k_hstep  segmented radix SELECT, most significant digit first: the threshold key theta, the count of
+//                            keys below it and m, the number of keys equal to theta that are taken
+//   k_hcount/k_gscan x2/k_hplace
+//                            stable compaction of those pairs into key_lo[1] / key_hi[1] / idx[1] (the LSD sort's second
+//                            buffer, unused here), at the distro's own offset
+//   k_hsort<WIDE>            one CTA per distro: stable LSD radix sort of its head over the key range [0, theta], then the
+//                            ranked queue + TotalValue of ranks [0, min(length, cap))
+struct HeadSel {
+  unsigned long long prefix;  // digits of theta fixed so far (theta after the last pass)
+  uint32_t need;              // ranks still to place among the keys that match the prefix (m after the last pass)
+  uint32_t below;             // keys below the prefix's range (the keys < theta after the last pass)
+  int32_t gpos;               // the distro's place in the general list: its row of `hist`
+  uint32_t all;               // 1: length <= cap, the head is the whole distro (theta = its largest key, no select pass)
+};
+struct DHead {
+  HeadSel* sel;      // [D]
+  uint32_t* hist;    // [general distros * 256] digit counts of the current pass
+  uint32_t* eq_sum;  // [NT] keys == theta per tile, then the tile's exclusive offset (G.tile_sum does the same for keys < theta)
+  int32_t cap;
+};
+constexpr int kHeadCap = EVG_PERSISTED_QUEUE_CAP;
+constexpr int kHsThreads = 1024, kHsWarps = kHsThreads / 32;
+constexpr int kHsChunks = (kHeadCap + kHsThreads - 1) / kHsThreads;  // 32-item chunks per warp
+static_assert(kHeadCap < 65536, "head positions are 16-bit");
+
+__device__ __forceinline__ unsigned long long gen_key(const DGen& G, int b, int64_t p, bool wide) {
+  unsigned long long k = G.key_lo[b][p];
+  if (wide) k |= (unsigned long long)G.key_hi[b][p] << 32;
+  return k;
+}
+
+__global__ void __launch_bounds__(256) k_hinit(DDistros D, DGen G, DHead H, const int32_t* __restrict__ general_list) {
+  H.hist[blockIdx.x * 256 + threadIdx.x] = 0u;
+  if (threadIdx.x == 0) {
+    const int d = general_list[blockIdx.x];
+    const int64_t n = D.task_off[d + 1] - D.task_off[d];
+    HeadSel s;
+    s.all = n <= H.cap ? 1u : 0u;
+    s.prefix = s.all ? G.vmm[2 * d] - G.vmm[2 * d + 1] : 0ull;
+    s.need = uint32_t(min(n, int64_t(H.cap))); s.below = 0u; s.gpos = int32_t(blockIdx.x);
+    H.sel[d] = s;
+  }
+}
+
+// The eight keys of slots t8 .. t8+7 (t8 a multiple of four: 128-bit loads inside [lo, hi)); bit m of the result: slot
+// t8+m holds a key of the distro.
+__device__ __forceinline__ uint32_t head_keys8(const DGen& G, int64_t t8, int64_t lo, int64_t hi, bool wide, unsigned long long key[8]) {
+  if (t8 >= lo && t8 + 7 < hi) {
+    const uint4 a = *reinterpret_cast<const uint4*>(G.key_lo[0] + t8), b = *reinterpret_cast<const uint4*>(G.key_lo[0] + t8 + 4);
+    const uint32_t l[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+    uint32_t u[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    if (wide) {
+      const uint4 c = *reinterpret_cast<const uint4*>(G.key_hi[0] + t8), e = *reinterpret_cast<const uint4*>(G.key_hi[0] + t8 + 4);
+      u[0] = c.x; u[1] = c.y; u[2] = c.z; u[3] = c.w; u[4] = e.x; u[5] = e.y; u[6] = e.z; u[7] = e.w;
+    }
+#pragma unroll
+    for (int m = 0; m < 8; m++) key[m] = l[m] | ((unsigned long long)u[m] << 32);
+    return 0xFFu;
+  }
+  uint32_t ok = 0;
+#pragma unroll
+  for (int m = 0; m < 8; m++) {
+    const int64_t p = t8 + m;
+    const bool in = p >= lo && p < hi;
+    key[m] = in ? gen_key(G, 0, p, wide) : 0ull;
+    ok |= uint32_t(in) << m;
+  }
+  return ok;
+}
+
+// Pass j (most significant digit first): per tile, the digits of the keys that match the prefix fixed so far.  Thread q
+// counts its 8 consecutive keys run by run: skewed values put most keys of a tile in a handful of top digits, and one
+// shared atomic per key would serialise on those few counters.
+__global__ void __launch_bounds__(256) k_hhist(int j, DDistros D, DGen G, DHead H) {
+  if (j >= *G.maxpass) return;
+  int d, cnt; int64_t seg, lo; bool wide;
+  const int tile = int(blockIdx.x + G.tile0);
+  if (!gen_tile(D, G, tile, j, &d, &seg, &lo, &cnt, &wide)) return;
+  const int shift = 8 * (gen_npass(gen_bits(G, d)) - 1 - j);
+  const HeadSel s = H.sel[d];
+  if (s.all) return;
+  const unsigned long long want = j == 0 ? 0ull : s.prefix >> (shift + 8);
+  __shared__ uint32_t h[256];
+  h[threadIdx.x] = 0;
+  __syncthreads();
+  unsigned long long key[8];
+  const uint32_t ok = head_keys8(G, G.tile_start[tile] + 8 * int64_t(threadIdx.x), lo, lo + cnt, wide, key);
+  uint32_t run_dg = 256u, run_n = 0;
+#pragma unroll
+  for (int m = 0; m < 8; m++) {
+    const bool take = ((ok >> m) & 1u) && (j == 0 || (key[m] >> (shift + 8)) == want);
+    const uint32_t dg = take ? uint32_t(key[m] >> shift) & 255u : 256u;
+    if (dg != run_dg && dg < 256u) {
+      if (run_n) atomicAdd(&h[run_dg], run_n);
+      run_dg = dg; run_n = 0;
+    }
+    run_n += take;
+  }
+  if (run_n) atomicAdd(&h[run_dg], run_n);
+  __syncthreads();
+  if (h[threadIdx.x]) atomicAdd(&H.hist[s.gpos * 256 + threadIdx.x], h[threadIdx.x]);
+}
+
+// Pass j, one block per distro, thread = digit: the digit at which the running count reaches `need` extends the prefix.
+__global__ void __launch_bounds__(256) k_hstep(int j, const int32_t* __restrict__ general_list, DGen G, DHead H) {
+  if (j >= *G.maxpass) return;
+  const int d = general_list[blockIdx.x];
+  const int np = gen_npass(gen_bits(G, d));
+  if (j >= np || H.sel[d].all) return;
+  const int shift = 8 * (np - 1 - j);
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  uint32_t* h = H.hist + blockIdx.x * 256;
+  const uint32_t c = h[tid];
+  h[tid] = 0u;  // ready for the next pass
+  const uint32_t need = H.sel[d].need;
+  __shared__ uint32_t sw[8];
+  uint32_t inc = c;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) { const uint32_t x = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += x; }
+  if (lane == 31) sw[warp] = inc;
+  __syncthreads();
+#pragma unroll
+  for (int w = 0; w < 8; w++) inc += w < warp ? sw[w] : 0u;
+  const uint32_t excl = inc - c;
+  if (excl < need && need <= inc) {  // exactly one digit: the keys matching the prefix number at least `need`
+    HeadSel& s = H.sel[d];
+    s.prefix |= (unsigned long long)tid << shift;
+    s.below += excl;
+    s.need = need - excl;
+  }
+}
+
+__device__ __forceinline__ bool head_tile(const DDistros& D, const DGen& G, int tile, int* d, int64_t* base, int64_t* lo, int64_t* hi) {
+  *d = G.tile_distro[tile];
+  *base = D.task_off[*d];
+  *lo = max(G.tile_start[tile], *base);
+  *hi = min(G.tile_start[tile] + kGTile, D.task_off[*d + 1]);
+  return gen_bits(G, *d) > 32;
+}
+
+// Per tile: keys < theta into G.tile_sum, keys == theta into H.eq_sum (k_gscan turns both into offsets).
+__global__ void __launch_bounds__(256) k_hcount(DDistros D, DGen G, DHead H) {
+  const int tile = int(blockIdx.x + G.tile0);
+  int d; int64_t base, lo, hi;
+  const bool wide = head_tile(D, G, tile, &d, &base, &lo, &hi);
+  const unsigned long long theta = H.sel[d].prefix;
+  uint32_t lt = 0, eq = 0;
+  for (int64_t p = lo + threadIdx.x; p < hi; p += 256) {
+    const unsigned long long key = gen_key(G, 0, p, wide);
+    lt += key < theta;
+    eq += key == theta;
+  }
+  lt = __reduce_add_sync(0xffffffffu, lt);
+  eq = __reduce_add_sync(0xffffffffu, eq);
+  __shared__ uint32_t sl[8], se[8];
+  if ((threadIdx.x & 31) == 0) { sl[threadIdx.x >> 5] = lt; se[threadIdx.x >> 5] = eq; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    uint32_t a = 0, b = 0;
+    for (int w = 0; w < 8; w++) { a += sl[w]; b += se[w]; }
+    G.tile_sum[tile] = a;
+    H.eq_sum[tile] = b;
+  }
+}
+
+// Per tile, thread q owns 8 consecutive slots (buffer order = thread order): a pair is taken when its key is below theta
+// or it is one of the first m keys equal to theta; its head position is the number of taken pairs before it.
+__global__ void __launch_bounds__(256) k_hplace(DDistros D, DGen G, DHead H) {
+  const int tile = int(blockIdx.x + G.tile0);
+  int d; int64_t base, lo, hi;
+  const bool wide = head_tile(D, G, tile, &d, &base, &lo, &hi);
+  const HeadSel s = H.sel[d];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int64_t t8 = G.tile_start[tile] + 8 * int64_t(tid);
+  unsigned long long key[8];
+  const uint32_t ok = head_keys8(G, t8, lo, hi, wide, key);
+  uint32_t n_lt = 0, n_eq = 0;
+#pragma unroll
+  for (int m = 0; m < 8; m++) {
+    n_lt += ((ok >> m) & 1u) && key[m] < s.prefix;
+    n_eq += ((ok >> m) & 1u) && key[m] == s.prefix;
+  }
+  const uint32_t mine = n_lt | (n_eq << 16);  // at most 2048 of each per tile
+  uint32_t inc = mine;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) { const uint32_t x = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += x; }
+  __shared__ uint32_t sw[8];
+  if (lane == 31) sw[warp] = inc;
+  __syncthreads();
+#pragma unroll
+  for (int w = 0; w < 8; w++) inc += w < warp ? sw[w] : 0u;
+  const uint32_t ex = inc - mine;
+  uint32_t plt = G.tile_sum[tile] + (ex & 0xFFFFu), peq = H.eq_sum[tile] + (ex >> 16);
+#pragma unroll
+  for (int m = 0; m < 8; m++) {
+    const int64_t p = t8 + m;
+    if (!((ok >> m) & 1u)) continue;
+    uint32_t pos;
+    if (key[m] < s.prefix) pos = plt++ + min(peq, s.need);
+    else if (key[m] == s.prefix && peq < s.need) pos = plt + peq++;
+    else continue;
+    G.key_lo[1][base + pos] = uint32_t(key[m]);
+    if (wide) G.key_hi[1][base + pos] = uint32_t(key[m] >> 32);
+    G.idx[1][base + pos] = G.idx[0][p];
+  }
+}
+
+// One CTA per general-path distro whose head keys need (WIDE) or do not need a second word.  The head's positions are
+// sorted, not the pairs: per pass, warp w ranks its contiguous slice of the current permutation chunk by chunk (MATCH
+// on the digit, the group's first lane bumps the warp's digit counter), thread = digit turns the warp counters into
+// offsets, and the positions are scattered into the other permutation.
+template <bool WIDE>
+__global__ void __launch_bounds__(kHsThreads, 1) k_hsort(const int32_t* __restrict__ general_list, DDistros D, DGen G, DHead H,
+                                                     int32_t* __restrict__ order, int64_t* __restrict__ total_value) {
+  const int d = general_list[blockIdx.x];
+  const HeadSel s = H.sel[d];
+  const int bits = s.prefix == 0ull ? 0 : 64 - __clzll((long long)s.prefix);  // head keys lie in [0, theta]
+  if ((bits > 32) != WIDE) return;
+  const int np = (bits + 7) >> 3;
+  const uint32_t k = s.below + s.need;
+  const int64_t base = D.task_off[d];
+  extern __shared__ __align__(16) unsigned char hs_smem[];
+  uint32_t (*wcnt)[256] = reinterpret_cast<uint32_t (*)[256]>(hs_smem);
+  uint32_t* s_lo = reinterpret_cast<uint32_t*>(hs_smem + sizeof(uint32_t) * kHsWarps * 256);
+  uint32_t* s_hi = s_lo + kHeadCap;  // WIDE only
+  uint16_t* perm0 = reinterpret_cast<uint16_t*>(s_lo + (WIDE ? 2 : 1) * kHeadCap);
+  uint16_t* perm1 = perm0 + kHeadCap;
+  __shared__ uint32_t s_wsum[8];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  for (uint32_t i = tid; i < k; i += kHsThreads) {
+    s_lo[i] = G.key_lo[1][base + i];
+    if (WIDE) s_hi[i] = G.key_hi[1][base + i];
+    perm0[i] = uint16_t(i);
+  }
+  const unsigned lt = (1u << lane) - 1u;
+  uint16_t* cur = perm0;
+  uint16_t* nxt = perm1;
+  for (int pass = 0; pass < np; pass++) {
+    const int sh = (8 * pass) & 31;
+    const uint32_t* src = (WIDE && pass >= 4) ? s_hi : s_lo;
+    for (int q = tid; q < kHsWarps * 256; q += kHsThreads) wcnt[q >> 8][q & 255] = 0u;
+    __syncthreads();
+    uint32_t dr[kHsChunks];  // digit (256 = no item) | rank inside the warp's slice << 9
+#pragma unroll
+    for (int c = 0; c < kHsChunks; c++) {
+      const uint32_t i = uint32_t((warp * kHsChunks + c) * 32 + lane);
+      const uint32_t dg = i < k ? (src[cur[i]] >> sh) & 255u : 256u;
+      const unsigned peers = __match_any_sync(0xffffffffu, dg);
+      const int lead = __ffs(peers) - 1;
+      uint32_t b = 0;
+      if (lane == lead && dg < 256u) { b = wcnt[warp][dg]; wcnt[warp][dg] = b + uint32_t(__popc(peers)); }
+      b = __shfl_sync(0xffffffffu, b, lead) + uint32_t(__popc(peers & lt));
+      dr[c] = dg | (b << 9);
+      __syncwarp();
+    }
+    __syncthreads();
+    uint32_t tot = 0;
+    if (tid < 256) {
+#pragma unroll
+      for (int w = 0; w < kHsWarps; w++) tot += wcnt[w][tid];
+      uint32_t inc = tot;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) { const uint32_t y = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += y; }
+      if (lane == 31) s_wsum[warp] = inc;
+      tot = inc - tot;  // exclusive inside the warp
+    }
+    __syncthreads();
+    if (tid < 256) {
+      uint32_t run = tot;
+      for (int w = 0; w < warp; w++) run += s_wsum[w];
+#pragma unroll
+      for (int w = 0; w < kHsWarps; w++) { const uint32_t y = wcnt[w][tid]; wcnt[w][tid] = run; run += y; }
+    }
+    __syncthreads();
+#pragma unroll
+    for (int c = 0; c < kHsChunks; c++) {
+      const uint32_t dg = dr[c] & 511u;
+      if (dg < 256u) nxt[wcnt[warp][dg] + (dr[c] >> 9)] = cur[(warp * kHsChunks + c) * 32 + lane];
+    }
+    __syncthreads();
+    uint16_t* t = cur; cur = nxt; nxt = t;
+  }
+  __syncthreads();
+  const unsigned long long vmax_ord = G.vmm[2 * d];
+  for (uint32_t r = tid; r < k; r += kHsThreads) {
+    const uint32_t p = cur[r];
+    unsigned long long key = s_lo[p];
+    if (WIDE) key |= (unsigned long long)s_hi[p] << 32;
+    order[base + r] = int32_t(G.idx[1][base + p]);
+    total_value[base + r] = unord_i64(vmax_ord - key);
+  }
+}
+template <bool WIDE>
+constexpr size_t hsort_smem() { return sizeof(uint32_t) * kHsWarps * 256 + sizeof(uint32_t) * kHeadCap * (WIDE ? 2 : 1) + sizeof(uint16_t) * 2 * kHeadCap; }

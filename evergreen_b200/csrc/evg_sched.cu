@@ -503,15 +503,17 @@ __global__ void __launch_bounds__(256) k_dur_final(DDur X, evg_duration_stat* ou
 }
 
 // The 13-field SortingValueBreakdown of the unit each ranked task was emitted
-// from (planner.go:472-476, model/task/task.go:3990-4038); both paths.
+// from (planner.go:472-476, model/task/task.go:3990-4038); both paths.  Row j of `breakdown` is rank j - row_off[d]
+// of the distro d with row_off[d] <= j < row_off[d + 1]: row_off = task_off gives every rank, the head offsets of
+// evg_run_resident_head the first min(length, cap).
 __global__ void __launch_bounds__(256) k_breakdown(DTasks T, DDistros D, DWork W, const URec* rec, int64_t now, int any_complex,
-                                                   const int32_t* order, int64_t* breakdown) {
+                                                   const int32_t* order, const int64_t* row_off, int64_t n_rows, int64_t* breakdown) {
   if (*W.err) return;
   const int64_t t = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
-  const int d = block_find_distro(D.task_off, D.n, t, T.n);
+  const int d = block_find_distro(row_off, D.n, t, n_rows);
   if (d < 0) return;
   const int64_t base = D.task_off[d];
-  const int64_t g = base + order[t];
+  const int64_t g = base + order[base + t - row_off[d]];
   UnitAcc a;
   acc_init(a);
   const uint32_t bp = any_complex ? W.best_pair[g] : kInactive;
@@ -850,9 +852,13 @@ struct evg_ctx {
   cudaEvent_t ev_h[kMaxChunks] = {}, ev_c[kMaxChunks] = {};
   int general_complex = 0;
   int64_t Tgc = 0;  // tasks in general-path distros that can hold multi-member units (work-list capacity)
+  int64_t max_general = 0;  // tasks in the longest general-path distro
   DevBuf b_kv, b_vmm, b_klo[2], b_khi[2], b_ix[2], b_e, b_tilesum, b_gmisc;
   DevBuf b_tiledistro, b_tilestart, b_dtileoff, b_tilehist, b_clist, b_rec, b_tie, b_hlist, b_usum, b_upd;
   DevBuf b_qinfo, b_ginfo, b_order, b_tv, b_bd;
+  DevBuf b_hsel, b_hhist, b_heq, b_hoff;  // evg_run_resident_head: selection state, digit counts, tile counts, head row offsets
+  int32_t head_cap = 0;                   // 0: the last run ranked every task; else only the first min(length, head_cap)
+  std::vector<int64_t> h_headoff;         // [D+1] offsets of each distro's head rows (the breakdown rows of a head run)
   DevBuf b_hflags, b_hgid, b_hexp, b_hstd, b_hstart, b_hostoff, b_acfg, b_gs, b_result, b_status;
   bool bd_valid = false;
   evg_alloc_result* ext_result = nullptr;  // caller-owned send buffer (evg_bind_result_buffer)
@@ -893,6 +899,7 @@ int upload_tasks(evg_ctx* c, const evg_task_soa* t, const evg_distro_table* dt, 
   std::vector<int64_t> tile_start;
   std::vector<uint8_t> route(size_t(D) + 1, 0);
   int32_t n_general = 0;
+  int64_t max_general = 0;
   int general_complex = 0;
   int any_complex = E > 0 ? 1 : 0;
   int64_t Tgc = 0, Prec = 0;
@@ -952,6 +959,7 @@ int upload_tasks(evg_ctx* c, const evg_task_soa* t, const evg_distro_table* dt, 
       case 6: listC.push_back(d); route[d] = 1; break;
       default: {
         n_general++;
+        max_general = std::max(max_general, n);
         listG.push_back(d);
         if (gb > ga || cf.group_versions || de > 0) {
           general_complex = 1;
@@ -1088,6 +1096,8 @@ int upload_tasks(evg_ctx* c, const evg_task_soa* t, const evg_distro_table* dt, 
   c->t_pad = (T + 3) & ~int64_t(3);
   c->adopted = adopt;
   c->deps_resident = false;
+  if (c->head_cap > 0) c->bd_valid = false;  // a head run's breakdown rows are laid out for the previous table
+  c->head_cap = 0;
   c->Tgc = Tgc;
   c->max_groups = 0;
   for (int32_t d = 0; d < D; d++) c->max_groups = std::max(c->max_groups, dt->group_off[d + 1] - dt->group_off[d]);
@@ -1096,6 +1106,7 @@ int upload_tasks(evg_ctx* c, const evg_task_soa* t, const evg_distro_table* dt, 
   c->nA = int32_t(listA.size()); c->nB = int32_t(listB.size()); c->nC = int32_t(listC.size());
   c->nNA = int32_t(listNA.size()); c->nNB = int32_t(listNB.size()); c->nNC = int32_t(listNC.size());
   c->n_general = n_general;
+  c->max_general = max_general;
   c->general_complex = general_complex;
   CK(c->b_err.ensure(sizeof(int) * 4));
   CK(cudaMemsetAsync(c->b_err.p, 0, sizeof(int) * 4, s));
@@ -1309,7 +1320,7 @@ int prepare_general(evg_ctx* c, cudaStream_t s, int32_t d0, int32_t d1) {
 
 // The general path on stream `st` for the general-path distros listG[gfirst .. gfirst + gcount) (evg_plan_general.cuh).
 int run_general(evg_ctx* c, cudaStream_t st, const DTasks& dt, const DDistros& dd, const DWork& w, int64_t now, int32_t gfirst,
-                int32_t gcount) {
+                int32_t gcount, int32_t head_cap = 0) {
   if (gcount <= 0) return EVG_OK;
   DGen g = dgen(c);
   const int gc = c->general_complex;
@@ -1338,13 +1349,39 @@ int run_general(evg_ctx* c, cudaStream_t st, const DTasks& dt, const DDistros& d
   LAUNCH_ON(c, st, k_gplace, nt, 256, dd, w, g, gc);
   if (gc) LAUNCH_ON(c, st, k_gplace_disp, wl_grid, 256, dt, dd, w, g);
   if (c->timed) CK(cudaEventRecord(c->ev_sort0, st));  // the general path's segmented sort
-  for (int j = 0; j < 8; j++) {  // passes beyond the tick's longest key exit at once (*maxpass is device-side)
-    LAUNCH_ON(c, st, k_ghist, nt, 256, j, dd, g);
-    LAUNCH_ON(c, st, k_gdscan, unsigned(gcount), 1024, j, gl, g);
-    LAUNCH_ON(c, st, k_gscatter, nt, 256, j, dd, g);
+  // The select pays when it discards most of a distro.  When no general-path distro is longer than twice the cap, the
+  // tile-parallel full sort (whose first cap ranks are the head) beats one CTA per distro sorting nearly all of it
+  // (configs[4]: a 12 546-task distro and two dozen sparse-class ones).
+  if (head_cap == 0 || c->max_general <= 2 * int64_t(head_cap)) {
+    for (int j = 0; j < 8; j++) {  // passes beyond the tick's longest key exit at once (*maxpass is device-side)
+      LAUNCH_ON(c, st, k_ghist, nt, 256, j, dd, g);
+      LAUNCH_ON(c, st, k_gdscan, unsigned(gcount), 1024, j, gl, g);
+      LAUNCH_ON(c, st, k_gscatter, nt, 256, j, dd, g);
+    }
+    if (c->timed) CK(cudaEventRecord(c->ev_sort1, st));
+    LAUNCH_ON(c, st, k_gemit, nt, 256, dd, g, c->b_order.as<int32_t>(), c->b_tv.as<int64_t>());
+  } else {  // select + compaction + head sort; TotalValue by task in b_tv was last read by k_gplace_disp
+    DHead h;
+    h.sel = c->b_hsel.as<HeadSel>(); h.hist = c->b_hhist.as<uint32_t>(); h.eq_sum = c->b_heq.as<uint32_t>(); h.cap = head_cap;
+    LAUNCH_ON(c, st, k_hinit, unsigned(gcount), 256, dd, g, h, gl);
+    for (int j = 0; j < 8; j++) {
+      LAUNCH_ON(c, st, k_hhist, nt, 256, j, dd, g, h);
+      LAUNCH_ON(c, st, k_hstep, unsigned(gcount), 256, j, gl, g, h);
+    }
+    LAUNCH_ON(c, st, k_hcount, nt, 256, dd, g, h);
+    LAUNCH_ON(c, st, k_gscan, unsigned(gcount), 1024, g, gl);
+    DGen ge = g;
+    ge.tile_sum = h.eq_sum;
+    LAUNCH_ON(c, st, k_gscan, unsigned(gcount), 1024, ge, gl);
+    LAUNCH_ON(c, st, k_hplace, nt, 256, dd, g, h);
+    constexpr size_t b0 = hsort_smem<false>(), b1 = hsort_smem<true>();
+    CK(cudaFuncSetAttribute(k_hsort<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(b0)));
+    CK(cudaFuncSetAttribute(k_hsort<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(b1)));
+    k_hsort<false><<<unsigned(gcount), kHsThreads, b0, st>>>(gl, dd, g, h, c->b_order.as<int32_t>(), c->b_tv.as<int64_t>());
+    k_hsort<true><<<unsigned(gcount), kHsThreads, b1, st>>>(gl, dd, g, h, c->b_order.as<int32_t>(), c->b_tv.as<int64_t>());
+    c->launches += 2;
+    if (c->timed) CK(cudaEventRecord(c->ev_sort1, st));
   }
-  if (c->timed) CK(cudaEventRecord(c->ev_sort1, st));
-  LAUNCH_ON(c, st, k_gemit, nt, 256, dd, g, c->b_order.as<int32_t>(), c->b_tv.as<int64_t>());
   const int64_t g0 = c->h_groupoff[size_t(d_first)], g1 = c->h_groupoff[size_t(d_last) + 1];
   LAUNCH_ON(c, st, k_finalize_info, grid_for(std::max<int64_t>(d_last + 1 - d_first, g1 - g0), 256), 256, dd, w, d_first, d_last + 1, g0, g1);
   return EVG_OK;
@@ -1360,7 +1397,9 @@ int ensure_aux_streams(evg_ctx* c) {
   return EVG_OK;
 }
 
-int run_plan(evg_ctx* c, int64_t now, uint32_t opts) {
+// head_cap > 0 (evg_run_resident_head): general-path distros rank only their first min(length, head_cap) tasks, and
+// breakdown rows exist for those ranks only, at the offsets c->h_headoff / b_hoff.
+int run_plan(evg_ctx* c, int64_t now, uint32_t opts, int32_t head_cap = 0) {
   const int64_t T = c->T;
   const int32_t D = c->Dn;
   cudaStream_t s = c->stream;
@@ -1369,8 +1408,27 @@ int run_plan(evg_ctx* c, int64_t now, uint32_t opts) {
   DWork w = dwork(c);
   int64_t* bd = nullptr;
   c->bd_valid = false;
+  c->head_cap = head_cap;
+  const int64_t* bd_off = c->b_taskoff.as<int64_t>();
+  int64_t bd_rows = T;
+  if (head_cap > 0) {
+    if (c->n_general > 0) {
+      CK(c->b_hsel.ensure(sizeof(HeadSel) * size_t(D + 1)));
+      CK(c->b_hhist.ensure(sizeof(uint32_t) * 256 * size_t(c->n_general)));
+      CK(c->b_heq.ensure(sizeof(uint32_t) * size_t(c->NT + 1)));
+    }
+    if (opts & EVG_OPT_BREAKDOWN) {  // host work before the first launch: only when the rows are wanted
+      c->h_headoff.assign(size_t(D) + 1, 0);
+      for (int32_t d = 0; d < D; d++)
+        c->h_headoff[size_t(d) + 1] = c->h_headoff[size_t(d)] + std::min<int64_t>(c->h_taskoff[size_t(d) + 1] - c->h_taskoff[size_t(d)], head_cap);
+      bd_rows = c->h_headoff[size_t(D)];
+      CK(c->b_hoff.ensure(sizeof(int64_t) * size_t(D + 1)));
+      CK(cudaMemcpyAsync(c->b_hoff.p, c->h_headoff.data(), sizeof(int64_t) * size_t(D + 1), cudaMemcpyHostToDevice, s));
+      bd_off = c->b_hoff.as<int64_t>();
+    }
+  }
   if (opts & EVG_OPT_BREAKDOWN) {
-    CK(c->b_bd.ensure(sizeof(int64_t) * EVG_BD_N * size_t(T + 1)));
+    CK(c->b_bd.ensure(sizeof(int64_t) * EVG_BD_N * size_t(bd_rows + 1)));
     bd = c->b_bd.as<int64_t>();
     c->bd_valid = true;
   }
@@ -1434,14 +1492,15 @@ int run_plan(evg_ctx* c, int64_t now, uint32_t opts) {
   // --- stream 4: one warp per tiny distro
   if ((rc = launch_tiny(c, st(4), dt, dd, w, c->b_listW.as<int32_t>(), c->nW, now, bd ? 1 : 0)) != EVG_OK) return rc;
   // --- stream 5: the general path
-  if (general && (rc = run_general(c, st(5), dt, dd, w, now, 0, c->n_general)) != EVG_OK) return rc;
+  if (general && (rc = run_general(c, st(5), dt, dd, w, now, 0, c->n_general, head_cap)) != EVG_OK) return rc;
   if (fork) {
     for (int k = 0; k < evg_ctx::kAux; k++) {
       CK(cudaEventRecord(c->ev_join[k], c->s_aux[k]));
       CK(cudaStreamWaitEvent(s, c->ev_join[k], 0));
     }
   }
-  if (bd) LAUNCH(c, k_breakdown, grid_for(T, 256), 256, dt, dd, w, c->b_rec.as<URec>(), now, c->any_complex, c->b_order.as<int32_t>(), bd);
+  if (bd) LAUNCH(c, k_breakdown, grid_for(bd_rows, 256), 256, dt, dd, w, c->b_rec.as<URec>(), now, c->any_complex, c->b_order.as<int32_t>(),
+                 bd_off, bd_rows, bd);
   CK(cudaGetLastError());
   return EVG_OK;
 }
@@ -1492,7 +1551,8 @@ void evg_shutdown(evg_ctx* c) {
                    &c->b_listNC, &c->b_lptA, &c->b_lptB, &c->b_lptC, &c->b_lptNA, &c->b_lptNB, &c->b_lptNC, &c->b_punt, &c->b_puntcnt, &c->b_ca, &c->b_crk, &c->b_bestpair, &c->b_kv, &c->b_vmm,
                    &c->b_klo[0], &c->b_klo[1], &c->b_khi[0], &c->b_khi[1], &c->b_ix[0], &c->b_ix[1], &c->b_e, &c->b_tilesum,
                    &c->b_gmisc, &c->b_clist, &c->b_rec, &c->b_tie, &c->b_hlist, &c->b_usum, &c->b_upd, &c->b_tiledistro, &c->b_tilestart, &c->b_dtileoff, &c->b_tilehist,
-                   &c->b_qinfo, &c->b_ginfo, &c->b_order, &c->b_tv, &c->b_bd, &c->b_hflags, &c->b_hgid, &c->b_hexp, &c->b_hstd,
+                   &c->b_qinfo, &c->b_ginfo, &c->b_order, &c->b_tv, &c->b_bd,
+                   &c->b_hsel, &c->b_hhist, &c->b_heq, &c->b_hoff, &c->b_hflags, &c->b_hgid, &c->b_hexp, &c->b_hstd,
                    &c->b_hstart, &c->b_hostoff, &c->b_acfg, &c->b_gs, &c->b_result, &c->b_status};
   for (DevBuf* b : all) b->release();
   for (DevBuf& b : c->b_pf) b.release();
@@ -1633,10 +1693,33 @@ int evg_run_resident(evg_ctx* c, int64_t now_ns, uint32_t opts) {
   return EVG_OK;
 }
 
+int evg_run_resident_head(evg_ctx* c, int64_t now_ns, uint32_t opts, int32_t cap) {
+  if (!c) return fail(EVG_ERR_INVALID, "null context");
+  LOCK(c);
+  if (cap == 0) cap = EVG_PERSISTED_QUEUE_CAP;
+  if (cap < 1 || cap > EVG_PERSISTED_QUEUE_CAP) return fail(EVG_ERR_INVALID, "evg_run_resident_head: cap %d outside [1, %d]", cap, EVG_PERSISTED_QUEUE_CAP);
+  if (!c->have_tasks) return fail(EVG_ERR_STATE, "evg_run_resident_head before evg_upload");
+  CK(cudaSetDevice(c->device));
+  c->launches = 0;
+  c->timed = true;
+  c->general_timed = false;
+  CK(cudaEventRecord(c->ev_begin, c->stream));
+  int rc = run_plan(c, now_ns, opts, cap);
+  if (rc != EVG_OK) return rc;
+  if (c->have_hosts) {
+    rc = run_alloc(c, now_ns);
+    if (rc != EVG_OK) return rc;
+  }
+  CK(cudaEventRecord(c->ev_end, c->stream));
+  return EVG_OK;
+}
+
 int evg_download(evg_ctx* c, evg_plan_out* po, evg_alloc_out* ao) {
   if (!c) return fail(EVG_ERR_INVALID, "null context");
   LOCK(c);
   if (!c->have_tasks) return fail(EVG_ERR_STATE, "evg_download before evg_upload");
+  if (po && c->head_cap > 0 && (po->order || po->total_value || po->breakdown))
+    return fail(EVG_ERR_STATE, "the last run ordered only the first %d ranks of each distro: download them with evg_download_queue", c->head_cap);
   CK(cudaSetDevice(c->device));
   cudaStream_t s = c->stream;
   if (po) {
@@ -1681,12 +1764,26 @@ __global__ void __launch_bounds__(256) k_project_queue(DTasks T, DDistros D, con
   items[j] = q;
 }
 
-int evg_download_queue(evg_ctx* c, int32_t cap, int64_t* item_off, evg_queue_item* items, int64_t items_capacity) {
-  if (!c) return fail(EVG_ERR_INVALID, "null context");
-  LOCK(c);
+// Row j of `out`: the breakdown row of the same rank as TaskQueueItem row j, read at bd_off[d] + rank.
+__global__ void __launch_bounds__(256) k_project_breakdown(int32_t n_distros, const int64_t* __restrict__ item_off, int64_t n_items,
+                                                           const int64_t* __restrict__ bd_off, const int64_t* __restrict__ bd,
+                                                           int64_t* __restrict__ out) {
+  const int64_t j = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (j >= n_items) return;
+  const int d = find_distro(item_off, 0, n_distros - 1, j);
+  const int64_t* src = bd + (bd_off[d] + j - item_off[d]) * EVG_BD_N;
+#pragma unroll
+  for (int k = 0; k < EVG_BD_N; k++) out[j * EVG_BD_N + k] = src[k];
+}
+
+namespace {
+int download_queue(evg_ctx* c, int32_t cap, int64_t* item_off, evg_queue_item* items, int64_t* breakdown, int64_t items_capacity) {
   if (!c->have_tasks) return fail(EVG_ERR_STATE, "evg_download_queue before evg_upload");
   if (cap < 0 || !item_off) return fail(EVG_ERR_INVALID, "evg_download_queue: bad argument");
   if (cap == 0) cap = EVG_PERSISTED_QUEUE_CAP;
+  if (c->head_cap > 0 && cap > c->head_cap)
+    return fail(EVG_ERR_STATE, "evg_download_queue: cap %d exceeds the %d ranks the last run ordered", cap, c->head_cap);
+  if (breakdown && !c->bd_valid) return fail(EVG_ERR_STATE, "evg_download_queue_bd: the last run did not set EVG_OPT_BREAKDOWN");
   const int32_t D = c->Dn;
   item_off[0] = 0;
   for (int32_t d = 0; d < D; d++) item_off[d + 1] = item_off[d] + std::min<int64_t>(c->h_taskoff[d + 1] - c->h_taskoff[d], cap);
@@ -1702,8 +1799,30 @@ int evg_download_queue(evg_ctx* c, int32_t cap, int64_t* item_off, evg_queue_ite
                                                  c->b_tv.as<int64_t>(), c->b_rn1.as<evg_queue_item>());
   CK(cudaGetLastError());
   CK(cudaMemcpyAsync(items, c->b_rn1.p, sizeof(evg_queue_item) * size_t(n), cudaMemcpyDeviceToHost, s));
+  if (breakdown) {  // the breakdown rows of a head run sit at its head offsets, those of a full run at task_off
+    const int64_t* bd_off = c->head_cap > 0 ? c->b_hoff.as<int64_t>() : c->b_taskoff.as<int64_t>();
+    CK(c->b_rn2.ensure(sizeof(int64_t) * EVG_BD_N * size_t(n)));
+    k_project_breakdown<<<grid_for(n, 256), 256, 0, s>>>(D, c->b_rn0.as<int64_t>(), n, bd_off, c->b_bd.as<int64_t>(), c->b_rn2.as<int64_t>());
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(breakdown, c->b_rn2.p, sizeof(int64_t) * EVG_BD_N * size_t(n), cudaMemcpyDeviceToHost, s));
+  }
   CK(cudaStreamSynchronize(s));
   return EVG_OK;
+}
+}  // namespace
+
+int evg_download_queue(evg_ctx* c, int32_t cap, int64_t* item_off, evg_queue_item* items, int64_t items_capacity) {
+  if (!c) return fail(EVG_ERR_INVALID, "null context");
+  LOCK(c);
+  return download_queue(c, cap, item_off, items, nullptr, items_capacity);
+}
+
+int evg_download_queue_bd(evg_ctx* c, int32_t cap, int64_t* item_off, evg_queue_item* items, int64_t* breakdown,
+                          int64_t items_capacity) {
+  if (!c) return fail(EVG_ERR_INVALID, "null context");
+  LOCK(c);
+  if (!breakdown) return fail(EVG_ERR_INVALID, "evg_download_queue_bd: null breakdown");
+  return download_queue(c, cap, item_off, items, breakdown, items_capacity);
 }
 
 void* evg_device_result_ptr(evg_ctx* c) { return c ? (void*)c->result_ptr() : nullptr; }
@@ -1792,6 +1911,7 @@ static int plan_and_alloc_pipelined(evg_ctx* c, const evg_task_soa* t, const evg
   c->launches = 0;
   c->timed = false;
   c->bd_valid = false;
+  c->head_cap = 0;
   CK(cudaMemsetAsync(c->b_puntcnt.p, 0, sizeof(int32_t) * (evg_ctx::kMaxChunks + 2), s));
   // chunk boundaries: whole distros, about equal task counts
   const int n_chunks = int(std::min<int64_t>(evg_ctx::kMaxChunks, std::max<int64_t>(1, T / (1 << 20))));

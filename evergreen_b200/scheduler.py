@@ -166,10 +166,17 @@ class Engine:
     def run(self, now: int, opts: int = 0) -> None:
         L.check(self.lib.evg_run_resident(self.ctx, int(now), int(opts)))
 
-    def download(self, want_breakdown: bool = False, want_alloc: Optional[bool] = None):
+    def run_head(self, now: int, cap: int = 0, opts: int = 0) -> None:
+        """evg_run_resident_head: like run(), but only the first min(length, cap) ranks of every distro are ordered
+        (cap 0 = the 10 000 TaskQueue.Save keeps).  Read them with download_queue(); download() then serves the queue
+        info, group info and allocator result only (ranks=False)."""
+        L.check(self.lib.evg_run_resident_head(self.ctx, int(now), int(opts), int(cap)))
+
+    def download(self, want_breakdown: bool = False, want_alloc: Optional[bool] = None, ranks: bool = True):
+        """ranks=False leaves order / total_value out (they are not defined after run_head)."""
         T, D, G = self._n_tasks, self._n_distros, self._n_groups
         po = self._plan_output(T, D, G, want_breakdown)
-        ps = L.PlanOutStruct(L.ptr(po.order), L.ptr(po.total_value),
+        ps = L.PlanOutStruct(L.ptr(po.order) if ranks else None, L.ptr(po.total_value) if ranks else None,
                              L.ptr(po.breakdown) if want_breakdown else None, L.ptr(po.info), L.ptr(po.group_info))
         ao = None
         if want_alloc is None:
@@ -182,16 +189,22 @@ class Engine:
             L.check(self.lib.evg_download(self.ctx, C.byref(ps), None))
         return po, ao
 
-    def download_queue(self, cap: int = 0, task_off=None):
+    def download_queue(self, cap: int = 0, task_off=None, breakdown: bool = False):
         """evg_download_queue: (item_off, items) -- the TaskQueueItem rows of the first min(length, cap) ranks of every
-        distro (cap 0 = the reference's 10 000), projected on the device; only those rows cross PCIe."""
+        distro (cap 0 = the reference's 10 000), projected on the device; only those rows cross PCIe.  breakdown=True
+        (evg_download_queue_bd, after a run with EVG_OPT_BREAKDOWN): (item_off, items, breakdown rows (n, EVG_BD_N))."""
         D = self._n_distros
         item_off = self._out("queue_item_off", D + 1, np.int64)
         cap_eff = cap or L.EVG_PERSISTED_QUEUE_CAP
         n = self._n_tasks if task_off is None else int(np.minimum(np.diff(task_off), cap_eff).sum())
         items = self._out("queue_items", max(n, 1), L.QUEUE_ITEM_DTYPE)
-        L.check(self.lib.evg_download_queue(self.ctx, int(cap), L.ptr(item_off), L.ptr(items), int(max(n, 1))))
-        return item_off, items[: int(item_off[D])]
+        if not breakdown:
+            L.check(self.lib.evg_download_queue(self.ctx, int(cap), L.ptr(item_off), L.ptr(items), int(max(n, 1))))
+            return item_off, items[: int(item_off[D])]
+        bd = self._out("queue_breakdown", (max(n, 1), L.EVG_BD_N), np.int64)
+        L.check(self.lib.evg_download_queue_bd(self.ctx, int(cap), L.ptr(item_off), L.ptr(items), L.ptr(bd), int(max(n, 1))))
+        rows = int(item_off[D])
+        return item_off, items[:rows], bd[:rows]
 
     def bind_result_buffer(self, device_ptr: int, capacity_rows: int) -> None:
         """The allocator kernel writes evg_alloc_result rows straight into this device buffer
@@ -451,18 +464,43 @@ def persist_task_queues(batch: Sequence[Tuple[M.Distro, List[M.Task]]], now: int
     eng.run(now)
     po, _ = eng.download(want_alloc=False)
     item_off, items = eng.download_queue(cap, table.task_off)
+    return _task_queue_documents(batch, now, table, keys, po, item_off, items, None)
+
+
+def persist_task_queue_heads(batch: Sequence[Tuple[M.Distro, List[M.Task]]], now: int, *, engine: Optional[Engine] = None,
+                             dependency_db: Optional[Dict[str, M.Task]] = None, cap: int = 0) -> List[M.TaskQueue]:
+    """persist_task_queues through the head tick (evg_run_resident_head with EVG_OPT_BREAKDOWN): only the first
+    min(length, cap) ranks of every distro are ordered -- what PlanDistro persists (scheduler/wrapper.go:107-127) --
+    and every TaskQueueItem carries its full SortingValueBreakdown (task_queue_persister.go:33).  Tasks are stamped as
+    persist_task_queues stamps them."""
+    eng = engine or default_engine()
+    soa, table, keys = S.marshal_tasks(batch, now, dependency_db)
+    _upload_with_device_deps(eng, batch, soa, table, None, now, dependency_db)
+    eng.run_head(now, cap, L.EVG_OPT_BREAKDOWN)
+    po, _ = eng.download(want_alloc=False, ranks=False)
+    item_off, items, bd = eng.download_queue(cap, table.task_off, breakdown=True)
+    return _task_queue_documents(batch, now, table, keys, po, item_off, items, bd)
+
+
+def _task_queue_documents(batch, now, table, keys, po, item_off, items, bd) -> List[M.TaskQueue]:
+    """The TaskQueue documents of a planned tick from its queue info and projected rows; `bd` (breakdown rows of the
+    same ranks) or None: the breakdown then holds TotalValue only."""
     out = []
     for d, (distro, tasks) in enumerate(batch):
         ga, gb = int(table.group_off[d]), int(table.group_off[d + 1])
         info = _queue_info_from_rows(po.info[d], po.group_info[ga:gb], keys[d].group_names)
         incl = distro.dispatcher_settings.version == M.DISPATCHER_VERSION_REVISED_WITH_DEPENDENCIES
         queue = []
-        for row in items[int(item_off[d]):int(item_off[d + 1])]:
+        for j in range(int(item_off[d]), int(item_off[d + 1])):
+            row = items[j]
             t = tasks[int(row["task"])]
             met = bool(int(row["flags"]) & L.EVG_QI_DEPS_MET)
             if met or not incl:  # GetDistroQueueInfo stamps ExpectedDuration only on the tasks it counts (scheduler.go:98)
                 t.expected_duration = int(row["expected_ns"])
-            t.sorting_value_breakdown = M.SortingValueBreakdown(total_value=int(row["total_value"]))
+            if bd is None:
+                t.sorting_value_breakdown = M.SortingValueBreakdown(total_value=int(row["total_value"]))
+            else:
+                t.sorting_value_breakdown = M.SortingValueBreakdown.from_row(bd[j])  # planner.go:475
             queue.append(M.TaskQueueItem(
                 id=t.id, display_name=t.display_name, build_variant=t.build_variant,
                 revision_order_number=t.revision_order_number, requester=t.requester, revision=t.revision, project=t.project,

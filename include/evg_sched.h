@@ -321,6 +321,26 @@ typedef struct {
  * (scheduler/task_queue_persister.go:14-42, model/task_queue.go:216-219).  The upsert stays with the caller. */
 int evg_download_queue(evg_ctx* ctx, int32_t cap, int64_t* item_off, evg_queue_item* items, int64_t items_capacity);
 
+/* Like evg_run_resident, but only the first min(length, cap) ranks of every distro are ordered: what
+ * PersistTaskQueue / TaskQueue.Save keep (scheduler/task_queue_persister.go:14-55, model/task_queue.go:216-219), and
+ * all a PlanDistro caller reads of the plan besides len(plan) (scheduler/wrapper.go:107-127).  Distros above the
+ * on-chip capacity select their cap smallest keys instead of sorting every task (when the longest of them exceeds twice
+ * the cap; below that the full sort is faster and its first cap ranks are the head).
+ * cap: 0 means EVG_PERSISTED_QUEUE_CAP; otherwise 1 <= cap <= EVG_PERSISTED_QUEUE_CAP, else -EVG_ERR_INVALID.
+ * Queue info, group info and allocator results are the same as after evg_run_resident, and so is every rank below
+ * the cap.  opts: EVG_OPT_BREAKDOWN is honoured for those ranks only.  Afterwards evg_download with a non-NULL order,
+ * total_value or breakdown is -EVG_ERR_STATE (those rows are not defined past the cut), and so are evg_download_queue /
+ * evg_download_queue_bd with a cap above this one (cap 0 included when this one is below EVG_PERSISTED_QUEUE_CAP).
+ * The next evg_run_resident restores the full contract.  evg_general_timing_ms's sort_ms spans select, compaction and
+ * head sort. */
+int evg_run_resident_head(evg_ctx* ctx, int64_t now_ns, uint32_t opts, int32_t cap);
+
+/* evg_download_queue plus breakdown[rows * EVG_BD_N]: the full SortingValueBreakdown of each row, in the same order
+ * (the TaskQueueItem.SortingValueBreakdown PersistTaskQueue copies, task_queue_persister.go:33).  Works after either
+ * kind of run that set EVG_OPT_BREAKDOWN; -EVG_ERR_STATE otherwise. */
+int evg_download_queue_bd(evg_ctx* ctx, int32_t cap, int64_t* item_off, evg_queue_item* items,
+                          int64_t* breakdown, int64_t items_capacity);
+
 /* Device pointer to the resident evg_alloc_result[n_distros] vector, the
  * send buffer of the per-distro all-gather (SURVEY.md §8e). */
 void* evg_device_result_ptr(evg_ctx* ctx);
@@ -342,7 +362,8 @@ int evg_last_timing_ms(evg_ctx* ctx, float* total_ms, float* sort_ms);
 int evg_kernel_timing_ms(evg_ctx* ctx, float* out_ms, int32_t n);
 
 /* The general path's two big stages in the last evg_run_resident (ms, CUDA events on its stream): the per-task
- * pass k_gtask (reads every input column once) and the segmented radix sort (all passes). */
+ * pass k_gtask (reads every input column once) and the segmented radix sort (all passes); after
+ * evg_run_resident_head, the select, compaction and head sort that replace it. */
 int evg_general_timing_ms(evg_ctx* ctx, float* task_pass_ms, float* sort_ms);
 
 /* ---- dependency filter (SURVEY.md §8f.1: the next row after the planner/allocator path) ---- */
